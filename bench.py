@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (also writes the search state, see dump_outputs)
 
 Workload (config.workload = "C3"): 19x19 Go (wq), 1024 concurrent games per GPU, 800 sims/move,
 20-block x 256 dual net (F=18, FC=512, A'=362, DefaultConf batch 256), two random-init nets (agents A
@@ -126,6 +127,34 @@ def oracle_lib():
     return K.load(so)
 
 
+DUMP_GAMES = 64  # games in the --dump-outputs sample
+
+
+def dump_outputs(e, n_games, out_dir):
+    """What a caller reads back after the last timed wave (az_tree_dump, az_game_state), for a fixed, seeded sample of
+    games: visit count N, value sum W and prior P of every root child by move (pass last) in both agents' trees (zeros
+    where a tree has no such child or no root yet), and the board.  Written as DIR/<name>.npy, float32 / float64."""
+    games = np.sort(np.random.default_rng(0).choice(n_games, min(n_games, DUMP_GAMES), replace=False))
+    A1 = e.action_space + 1
+    visits = np.zeros((len(games), 2, A1), np.float64)
+    wsum = np.zeros((len(games), 2, A1), np.float32)
+    prior = np.zeros((len(games), 2, A1), np.float32)
+    board = np.zeros((len(games), e.cells), np.float32)
+    for i, g in enumerate(games.tolist()):
+        for t in (0, 1):
+            ch = e.tree_dump(g, t)
+            ch = ch[ch[:, 0] == 1]  # rows: depth, move, N, W bits, P bits, expanded, n_children
+            mv = np.where(ch[:, 1] == K.PASS, A1 - 1, ch[:, 1])
+            visits[i, t, mv] = ch[:, 2]
+            wsum[i, t, mv] = ch[:, 3].copy().view(np.float32)
+            prior[i, t, mv] = ch[:, 4].copy().view(np.float32)
+        board[i] = e.game_state(g)["board"]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("games", games.astype(np.float64)), ("root_visits", visits), ("root_value_sum", wsum),
+                    ("root_prior", prior), ("board", board)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def setup_nets(e, seed):
     e.net_init(0, seed + 100)
     e.net_init(1, seed + 101)
@@ -193,7 +222,12 @@ def main():
     ap.add_argument("--no-fast", action="store_true", help="skip the AZ_FLAG_FAST_TOWER arm")
     ap.add_argument("--fast-tower", action="store_true", help="run the main arm with AZ_FLAG_FAST_TOWER (experiments)")
     ap.add_argument("--cpu-steps", type=int, default=24)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the main arm's timed steps, write rank 0's search state for a fixed sample of games to "
+                         "DIR/<name>.npy (identical inputs from run to run: compare two builds output for output)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     w = dict(WORKLOADS[args.workload])
     if args.games:
         w["n_games"] = args.games
@@ -249,7 +283,7 @@ def main():
     ctx = dict(lib=lib, w=w, args=args, rank=rank, world=world, local_rank=local_rank, dist=dist, torch=torch, warmup=warmup)
     probe = probe_planes(w, 32)
     main_arm = selfplay_arm(ctx, flags=K.FLAG_FAST_TOWER if args.fast_tower else 0, do_e2e=not args.no_e2e, probe=probe,
-                            do_train=not args.no_train)
+                            do_train=not args.no_train, dump_dir=args.dump_outputs if rank == 0 else None)
     fast_arm = None
     if not args.no_fast and not args.fast_tower and world == 1:
         fast_arm = selfplay_arm(ctx, flags=K.FLAG_FAST_TOWER, do_e2e=False, probe=probe, do_train=False, steps=min(args.steps, 60))
@@ -366,9 +400,10 @@ def roofline_of(arm, w, peaks, peak_src):
                     "fraction of the bf16 peak tops out at %.3f" % (passes, pad, 1.0 / (passes * pad))}
 
 
-def selfplay_arm(ctx, flags, do_e2e, probe, do_train, steps=None):
+def selfplay_arm(ctx, flags, do_e2e, probe, do_train, steps=None, dump_dir=None):
     """One engine, one precision mode: warm-up, the timed region of `steps` MCTS waves, optionally the end-to-end ply and
-    the training / collective block, then the precision probe; the engine is closed before returning."""
+    the training / collective block, then the precision probe; the engine is closed before returning.  With `dump_dir`
+    the search state after the first timed region is written there (dump_outputs)."""
     lib, w, args, rank, world, local_rank = ctx["lib"], ctx["w"], ctx["args"], ctx["rank"], ctx["world"], ctx["local_rank"]
     dist, torch, warmup = ctx["dist"], ctx["torch"], ctx["warmup"]
     steps = steps or args.steps
@@ -421,6 +456,8 @@ def selfplay_arm(ctx, flags, do_e2e, probe, do_train, steps=None):
     e.profile(True)
     two_regions = e.profile(False)["kernel_kind"] == 5
     prof, clocks, cnt = timed_region(2 if two_regions else 1)
+    if dump_dir:  # here, not after a re-measure: the dumped state is always warm-up + `steps` waves from the opening
+        dump_outputs(e, n_games, dump_dir)
     bad = {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"}
     if bad & set(clocks.get("reasons", [])) and world == 1:  # rejected: re-measure once (timing rules)
         prof, clocks2, cnt = timed_region(2 if two_regions else 1)

@@ -1,10 +1,14 @@
 """bench.py's reference arm (`--impl reference`: the CPU oracle on the host cores) end to end on the small workload, and
 the arithmetic of its roofline helper: the keys the driver parses are there, the faithful rate (every evaluation padded
-to ActionSpace samples, meta.go:125-135) sits below the useful-work rate, rank > 0 prints nothing."""
+to ActionSpace samples, meta.go:125-135) sits below the useful-work rate, rank > 0 prints nothing; and, on the GPU, the
+search state --dump-outputs writes."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -37,6 +41,37 @@ def test_reference_arm_other_ranks_are_silent():
     r = _run(["--impl", "reference", "--workload", "C2", "--steps", "2", "--warmup", "3", "--gpus", "2"],
              env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_needs_the_b200_arm(tmp_path):
+    r = _run(["--impl", "reference", "--workload", "C2", "--steps", "2", "--dump-outputs", str(tmp_path / "d")])
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_after_exactly_the_timed_steps(tmp_path):
+    """--dump-outputs writes the search state after warm-up + `--steps` waves, float32/float64 within 64 MB, and the
+    same bytes on a repeat run with the same arguments."""
+    steps, warmup, games = 7, 3, 16
+    dumps = []
+    for i in range(2):
+        d = tmp_path / str(i)
+        r = _run(["--workload", "C2", "--games", str(games), "--steps", str(steps), "--warmup", str(warmup), "--no-e2e",
+                  "--no-cpu-baseline", "--no-train", "--no-fast", "--dump-outputs", str(d)])
+        assert r.returncode == 0, r.stderr[-500:]
+        assert json.loads(r.stdout)["steps"] == steps
+        dumps.append({f.stem: np.load(f) for f in d.iterdir()})
+    a, b = dumps
+    assert set(a) == {"games", "root_visits", "root_value_sum", "root_prior", "board"}
+    assert all(x.dtype in (np.float32, np.float64) for x in a.values()) and sum(x.nbytes for x in a.values()) <= 64 << 20
+    for k in a:
+        assert a[k].tobytes() == b[k].tobytes(), k
+    assert (a["games"] == np.arange(games)).all() and a["root_visits"].shape == (games, 2, 82)
+    # the first warm-up step is the root evaluation, every later one a simulation; a root child is born with one visit
+    v = a["root_visits"]
+    sims = np.where(v > 0, v - 1, 0).sum(axis=2).max(axis=1)
+    assert sims.max() == warmup + steps - 1, sims
+    assert (np.abs(a["root_prior"].sum(axis=2).max(axis=1) - 1) < 1e-3).all()
 
 
 def test_roofline_arithmetic():
